@@ -144,7 +144,8 @@ def build_pipe(device, degenerate_temporal: bool = False):
 
 
 def edit_clip(pipe, x0_dev, emb_src):
-    """One full clip edit through the reference-facing API: inversion with STORE, then edit_type='swap'. Returns final latents."""
+    """One full clip edit through the reference-facing API: inversion with STORE, then edit_type='swap'.  Returns the inverted latents
+    the edit starts from and the pipeline call's result dict."""
     from fatezero_b200 import controllers
     pipe.scheduler.set_timesteps(DDIM_STEPS)
     old = getattr(pipe, "store_controller", None)
@@ -164,7 +165,35 @@ def edit_clip(pipe, x0_dev, emb_src):
                num_inference_steps=DDIM_STEPS, clip_length=x0_dev.shape[2], guidance_scale=7.5, num_images_per_prompt=1, latents=inv[-1],
                uncond_embeddings_list=None, save_path=save_path, height=8 * CFG["size"], width=8 * CFG["size"], output_type="latent",
                use_inversion_attention=True, save_self_attention=False, **CFG["p2p"])
-    return out["sdimage_output"].images
+    return inv[-1], out
+
+
+FRAME_AXIS = {"inverted_latents": 2, "edited_latents": 2, "mask_list": 1}
+
+
+def dump_outputs(dirname, inv_latents, out, world, shard_frames):
+    """--dump-outputs: what one clip edit returned to its caller, as float32 DIR/<name>.npy (a few MB: the latents, plus the per-step
+    latent-blend masks of the configs that blend latents).  Inputs and weights are seeded, so two builds can be compared file by file.
+    N > 1: gathered on rank 0, the ranks' frames joined along the frame axis (--shard frames) or stacked as a leading clip axis."""
+    import numpy as np
+    import torch.distributed as dist
+    arrays = {"inverted_latents": inv_latents, "edited_latents": out["sdimage_output"].images}
+    if out["mask_list"]:
+        arrays["mask_list"] = torch.stack(out["mask_list"])
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = world * sum(a.nbytes for a in arrays.values())  # every rank holds equal shapes: all ranks decide alike, before the gather
+    if total > 64 << 20:
+        raise SystemExit(f"--dump-outputs: {total / 2**20:.1f} MiB exceeds the 64 MiB bound")
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, arrays)
+        arrays = {k: np.concatenate([p[k] for p in parts], axis=FRAME_AXIS[k]) if shard_frames else np.stack([p[k] for p in parts])
+                  for k in arrays}
+        if dist.get_rank() != 0:
+            return
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), a)
 
 
 def instrument(pipe, x0_dev, emb_src):
@@ -324,13 +353,15 @@ def run_gpu(args):
             ms = float(t.item())
         return ms
 
+    last = {}
+
     def step_resident():
-        edit_clip(pipe, x0_dev, emb_src)
+        last["inv"], last["out"] = edit_clip(pipe, x0_dev, emb_src)
 
     def step_e2e():
         xd = x0_host.to(device, non_blocking=True)
-        lat = edit_clip(pipe, xd, emb_src)
-        out_host.copy_(lat.float(), non_blocking=True)
+        _, out = edit_clip(pipe, xd, emb_src)
+        out_host.copy_(out["sdimage_output"].images.float(), non_blocking=True)
         torch.cuda.current_stream().synchronize()
 
     # W >= 3 (timing rule); with cuda_graphs=auto the first clip runs eagerly, the second is captured, the third is the first pure replay
@@ -345,6 +376,9 @@ def run_gpu(args):
     ms = timed(step_resident, args.steps)
     launches = _lib.kernel_launches - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:  # before the next pass reuses the buffers (graph replays write the same masks in place)
+        dump_outputs(args.dump_outputs, last["inv"], last["out"], world, shard_frames)
+    last.clear()
     ms_e2e = timed(step_e2e, args.steps)
     frames_total = FRAMES * (1 if (shard_frames or world == 1) else world) * args.steps
     value = frames_total / (ms / 1e3)
@@ -464,23 +498,17 @@ def run_reference(args):
         return
     cores = cpu_threads()
     torch.set_num_threads(cores)
-    F = int(os.environ.get("FZ_REF_FRAMES", CFG["frames"]))  # tests/test_bench_contract.py shrinks the sample; the driver never sets it
-    times = []
-    t_start = time.perf_counter()
-    budget = float(os.environ.get("FZ_REF_BUDGET_S", "150"))
-    for i in range(args.warmup + args.steps):
-        t_inv, t_edit = cpu_sample_seconds(F)
-        if i >= min(args.warmup, 1):  # at most one untimed pass: every pass costs the better part of a minute
-            times.append(t_inv + t_edit)
-        elapsed = time.perf_counter() - t_start
-        if times and (len(times) >= args.steps or elapsed + (elapsed / (i + 1)) > budget):
-            break
+    F = int(os.environ.get("FZ_REF_FRAMES", CFG["frames"]))  # fewer frames than the clip: a quick check of the arm, not its number
+    warmup = min(args.warmup, 1)  # at most one untimed pass: every pass costs the better part of a minute
+    for _ in range(warmup):
+        cpu_sample_seconds(F)
+    times = [sum(cpu_sample_seconds(F)) for _ in range(args.steps)]
     pair = sum(times) / len(times)
     value = F / (DDIM_STEPS * pair)  # frames/s of the sampled frames (== the clip's when F is the clip length)
     sample = (f"each step = 1 of 50 DDIM step pairs on all {F} frames (oracle port of the reference, fp32, {cores} threads), "
-              f"{len(times)} timed after {min(args.warmup, 1)} untimed; scaled linearly in steps only")
+              f"{len(times)} timed after {warmup} untimed; scaled linearly in steps only")
     line = dict(impl="reference", metric="edited frames/sec (512x512x8f, 50 DDIM steps: inversion + attention-fused edit)",
-                value=round(value, 6), unit="frames/s", n_gpus=int(os.environ.get("WORLD_SIZE", "1")), steps=len(times), warmup=min(args.warmup, 1),
+                value=round(value, 6), unit="frames/s", n_gpus=int(os.environ.get("WORLD_SIZE", "1")), steps=len(times), warmup=warmup,
                 ms_per_step=round(pair * 1e3 * DDIM_STEPS, 1), higher_is_better=True, scaling="strong", vs_baseline=None, dtype="f32",
                 data="synthetic", config=dict(workload=CFG["workload"], name=CFG["name"], frames=F, latent=f"{CFG['size']}x{CFG['size']}",
                                              ddim_steps=DDIM_STEPS, model_config=CFG["model_config"]),
@@ -492,7 +520,9 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="timed steps; a step is one full clip edit (50 inversion + 50 edit DDIM steps) in the GPU arm, one DDIM step pair "
+                         "(inversion + edit) on all frames in the reference arm")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="style", choices=sorted(CONFIGS), help="BASELINE.json configs #2..#5 (default: the metric's own)")
@@ -501,7 +531,12 @@ def main():
     ap.add_argument("--graphs", default="auto", choices=["auto", "off"])
     ap.add_argument("--shard", default="frames", choices=["clips", "frames"],
                     help="N > 1: the frames of ONE clip over the ranks (default, strong scaling) or independent clips per rank (replicas)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs")
     select_config(args.config)
     if args.impl == "reference":
         run_reference(args)

@@ -66,3 +66,19 @@ CASES = {
 GPU_CASES = [k for k, v in CASES.items() if v.get("gpu", True)]
 BIG_CASES = [k for k, v in CASES.items() if v.get("big")]
 SMALL_CASES = [k for k, v in CASES.items() if not v.get("big")]
+
+# host-side edit tables: tests/test_tables.py, pinned against the reference by oracle/make_ref_pins.py (ref_tables_clip)
+PROMPT_PAIRS = [
+    (SRC, "watercolor painting of " + SRC),
+    (SRC, "a Porsche car driving down a curvy road in the countryside"),
+    ("a silver jeep driving down a curvy road", "a red jeep driving down a curvy road"),
+    ("a cat sitting next to a mirror", "a silver cat sculpture sitting next to a mirror"),
+    ("a photorealistic squirrel eating a burger", "a photorealistic lion eating a burger"),
+    ("a bear walking", "a extraordinarily fluffy bear is walking"),
+]
+
+# the reference's sample logger: tests/test_boundary_logger.py, pinned by oracle/make_ref_pins.py (ref_logger)
+LOGGER_EDITS = [SRC, "watercolor painting of " + SRC]
+LOGGER_P2P = {0: dict(is_replace_controller=False, cross_replace_steps={"default_": 0.8}, self_replace_steps=0.9, blend_self_attention=True),
+              1: dict(is_replace_controller=False, cross_replace_steps={"default_": 0.8}, self_replace_steps=0.8,
+                      eq_params={"words": ["watercolor"], "values": [10, 10]})}  # config/style/jeep_watercolor.yaml:36-68

@@ -1,12 +1,15 @@
 """Drop-in boundary (SURVEY.md §8(b)): the reference's UNCHANGED `P2pSampleLogger.log_sample_images`
 (video_diffusion/pipelines/p2p_validation_loop.py:68-131) must be able to drive this repo's pipeline.
 
-Two halves, because the reference tree only exists in the build container and the GPU only on the GPU box:
-  * CPU, reference present: import the reference's logger THROUGH this repo's `video_diffusion` alias package (modules the alias does not
-    provide fall through to the reference tree), run `log_sample_images` against a recording pipeline, and bind every recorded call to
-    the signature of our `P2pDDIMSpatioTemporalPipeline.__call__` / `sd_ddim_pipeline` / `make_controller`;
+Two halves:
+  * CPU: the reference's logger, imported THROUGH this repo's `video_diffusion` alias package (modules the alias does not provide fall
+    through to the reference tree), ran `log_sample_images` against a recording pipeline (oracle/make_ref_pins.py, pinned in
+    tests/golden/ref_logger.json.gz); every recorded call must bind to the signature of our `sd_ddim_pipeline` / `make_controller`, and
+    the alias must still fall through for modules it does not provide;
   * GPU: the same call sequence (kwargs as recorded there, cited line by line) against the real CUDA pipeline with stub VAE / tokenizer."""
+import gzip
 import inspect
+import json
 import os
 import sys
 
@@ -16,13 +19,8 @@ import torch
 
 from _helpers import ROOT, build_product
 from fatezero_b200 import synth
+from oracle.cases import LOGGER_EDITS as EDITS, LOGGER_P2P as P2P, SRC
 
-REF = "/root/reference"
-SRC = "a silver jeep driving down a curvy road in the countryside"
-EDITS = [SRC, "watercolor painting of " + SRC]
-P2P = {0: dict(is_replace_controller=False, cross_replace_steps={"default_": 0.8}, self_replace_steps=0.9, blend_self_attention=True),
-       1: dict(is_replace_controller=False, cross_replace_steps={"default_": 0.8}, self_replace_steps=0.8,
-               eq_params={"words": ["watercolor"], "values": [10, 10]})}  # config/style/jeep_watercolor.yaml:36-68
 
 
 def logger_kwargs(idx, prompt, image, latents, save_dir, steps, clip_length):
@@ -34,55 +32,54 @@ def logger_kwargs(idx, prompt, image, latents, save_dir, steps, clip_length):
                 uncond_embeddings_list=None, save_path=save_dir, **cfg)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "video_diffusion")), reason="reference tree only exists in the build container")
+def _replay(v, save_dir):
+    """A recorded keyword value of ref_logger.json.gz back as the object the reference logger passed."""
+    if isinstance(v, dict) and "__tensor__" in v:
+        return torch.zeros(v["__tensor__"])
+    if isinstance(v, dict) and "__generator__" in v:
+        return torch.Generator(device=v["__generator__"]).manual_seed(0)
+    if isinstance(v, dict) and "__save_dir__" in v:
+        return save_dir
+    return v
+
+
 def test_unchanged_reference_logger_binds_to_our_pipeline(tmp_path):
+    """The pipeline calls of the reference's log_sample_images (pinned by `python -m oracle.make_ref_pins ref_logger`) bind to our
+    pipeline and make_controller, and the alias package still lets the reference's own modules (the logger among them) fall through."""
+    fake = tmp_path / "ref" / "video_diffusion" / "pipelines"
+    fake.mkdir(parents=True)
+    (fake / "p2p_validation_loop.py").write_text("P2pSampleLogger = 'reference logger'\n")
     code = r'''
-import inspect, json, sys, types
-import numpy as np, torch
-from PIL import Image
-sys.path.insert(0, %(root)r); sys.path.insert(0, %(root)r + "/oracle/shim"); sys.path.append(%(ref)r)
+import sys
+sys.path.insert(0, %(root)r); sys.path.append(%(ref)r)
 import video_diffusion                                        # THIS repo's alias package ...
-from video_diffusion.pipelines.p2p_validation_loop import P2pSampleLogger   # ... falling through to the reference's own file
-import video_diffusion.pipelines.p2p_validation_loop as m
+import video_diffusion.pipelines.p2p_validation_loop as m    # ... falling through to the reference's own file
 assert m.__file__.startswith(%(ref)r), m.__file__
 from video_diffusion.pipelines.p2p_ddim_spatial_temporal import P2pDDIMSpatioTemporalPipeline as Ours
 assert Ours.__module__ == "fatezero_b200.pipeline", Ours.__module__
-from fatezero_b200 import controllers
-
-calls = []
-class Recorder:
-    @staticmethod
-    def numpy_to_pil(x):
-        return Ours.numpy_to_pil(x)
-    def __call__(self, **kw):
-        calls.append(kw)
-        frames = [Image.fromarray(np.zeros((16, 16, 3), np.uint8)) for _ in range(2)]
-        return {"sdimage_output": types.SimpleNamespace(images=[frames]), "attention_output": None, "mask_list": None}
-
-p2p = %(p2p)r
-lg = P2pSampleLogger(editing_prompts=%(edits)r, clip_length=2, logdir=%(tmp)r, num_inference_steps=3, guidance_scale=7.5, sample_seeds=[0],
-                     prompt2prompt_edit=True, p2p_config=p2p, use_inversion_attention=True, source_prompt=%(src)r)
-lg.log_sample_images(pipeline=Recorder(), device=torch.device("cpu"), step=0, image=torch.zeros(2, 3, 16, 16), latents=torch.zeros(1, 4, 2, 4, 4),
-                     save_dir=%(tmp)r)
-assert len(calls) == 2
-sig_call = inspect.signature(Ours.sd_ddim_pipeline)
-mk = inspect.signature(controllers.make_controller)
-for kw in calls:
-    assert kw["edit_type"] == "swap" and kw["use_inversion_attention"] is True and kw["save_self_attention"] is False
-    bound = sig_call.bind(None, controller=None, **kw)     # **args swallows what sd_ddim_pipeline does not name (p2p_ddim_spatial_temporal.py:280)
-    # p2preplace_edit (p2p_ddim_spatial_temporal.py:172-222) forwards these keys to make_controller under these names
-    mk.bind(None, [kw["source_prompt"], kw["prompt"]], NUM_DDIM_STEPS=kw["num_inference_steps"], is_replace_controller=kw.get("is_replace_controller", True),
-            cross_replace_steps=kw["cross_replace_steps"], self_replace_steps=kw["self_replace_steps"], blend_words=kw.get("blend_words"),
-            equilizer_params=kw.get("eq_params"), additional_attention_store=None, use_inversion_attention=kw["use_inversion_attention"],
-            blend_th=kw.get("blend_th", (0.3, 0.3)), blend_self_attention=kw.get("blend_self_attention"), blend_latents=kw.get("blend_latents"),
-            save_path=kw.get("save_path"), save_self_attention=kw.get("save_self_attention", True), disk_store=kw.get("disk_store", False))
-print(json.dumps(sorted(calls[1].keys())))
-''' % dict(root=ROOT, ref=REF, p2p=P2P, edits=EDITS, tmp=str(tmp_path / "log"), src=SRC)
+print("OK")
+''' % dict(root=ROOT, ref=str(tmp_path / "ref"))
     import subprocess
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-3000:]
-    import json
-    recorded = set(json.loads(r.stdout.strip().splitlines()[-1]))
+    assert r.returncode == 0 and "OK" in r.stdout, r.stdout[-1500:] + r.stderr[-3000:]
+
+    from fatezero_b200 import P2pDDIMSpatioTemporalPipeline as Ours
+    from fatezero_b200 import controllers
+    g = json.load(gzip.open(os.path.join(ROOT, "tests", "golden", "ref_logger.json.gz")))
+    calls = [{k: _replay(v, str(tmp_path)) for k, v in kw.items()} for kw in g["calls"]]
+    assert len(calls) == 2
+    sig_call = inspect.signature(Ours.sd_ddim_pipeline)
+    mk = inspect.signature(controllers.make_controller)
+    for kw in calls:
+        assert kw["edit_type"] == "swap" and kw["use_inversion_attention"] is True and kw["save_self_attention"] is False
+        sig_call.bind(None, controller=None, **kw)     # **args swallows what sd_ddim_pipeline does not name (p2p_ddim_spatial_temporal.py:280)
+        # p2preplace_edit (p2p_ddim_spatial_temporal.py:172-222) forwards these keys to make_controller under these names
+        mk.bind(None, [kw["source_prompt"], kw["prompt"]], NUM_DDIM_STEPS=kw["num_inference_steps"], is_replace_controller=kw.get("is_replace_controller", True),
+                cross_replace_steps=kw["cross_replace_steps"], self_replace_steps=kw["self_replace_steps"], blend_words=kw.get("blend_words"),
+                equilizer_params=kw.get("eq_params"), additional_attention_store=None, use_inversion_attention=kw["use_inversion_attention"],
+                blend_th=kw.get("blend_th", (0.3, 0.3)), blend_self_attention=kw.get("blend_self_attention"), blend_latents=kw.get("blend_latents"),
+                save_path=kw.get("save_path"), save_self_attention=kw.get("save_self_attention", True), disk_store=kw.get("disk_store", False))
+    recorded = set(calls[1].keys())
     mine = set(logger_kwargs(1, EDITS[1], None, None, None, 3, 2).keys())
     assert recorded == mine, (recorded ^ mine)   # the GPU half below replays exactly the keyword set the reference logger sends
 

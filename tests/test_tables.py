@@ -1,7 +1,7 @@
-"""Host-side edit tables: product (fatezero_b200.tables / controllers) == oracle restatement == reference (when present)."""
+"""Host-side edit tables: product (fatezero_b200.tables / controllers) == oracle restatement == reference (pinned)."""
+import gzip
+import json
 import os
-import subprocess
-import sys
 
 import pytest
 import torch
@@ -9,16 +9,7 @@ import torch
 from _helpers import ROOT
 from fatezero_b200 import controllers, synth, tables
 from oracle import fz_oracle as fo
-from oracle.cases import CASES, SRC
-
-PROMPT_PAIRS = [
-    (SRC, "watercolor painting of " + SRC),
-    (SRC, "a Porsche car driving down a curvy road in the countryside"),
-    ("a silver jeep driving down a curvy road", "a red jeep driving down a curvy road"),
-    ("a cat sitting next to a mirror", "a silver cat sculpture sitting next to a mirror"),
-    ("a photorealistic squirrel eating a burger", "a photorealistic lion eating a burger"),
-    ("a bear walking", "a extraordinarily fluffy bear is walking"),
-]
+from oracle.cases import CASES, PROMPT_PAIRS
 
 
 @pytest.mark.parametrize("src,tgt", PROMPT_PAIRS)
@@ -77,47 +68,41 @@ def test_make_controller_tables(name, tmp_path):
             assert (ctrl.latent_blend.start_blend, ctrl.latent_blend.end_blend) == plan.lat_window
 
 
-REF = "/root/reference"
+GOLDEN_TABLES = os.path.join(ROOT, "tests", "golden", "ref_tables_clip.json.gz")  # python -m oracle.make_ref_pins ref_tables_clip
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
+class ReplayTokenizer:
+    """The real CLIP BPE tokenizer's answers, as recorded while the reference computed the pinned tables."""
+
+    def __init__(self, rec):
+        self.encoded, self.decoded = rec["encode"], rec["decode"]
+
+    def encode(self, text):
+        assert text in self.encoded, f"encode({text!r}) was not recorded: regenerate the pin"
+        return list(self.encoded[text])
+
+    def decode(self, ids):
+        assert len(ids) == 1 and str(int(ids[0])) in self.decoded, f"decode({ids!r}) was not recorded: regenerate the pin"
+        return self.decoded[str(int(ids[0]))]
+
+
 def test_tables_match_reference_with_clip_tokenizer():
-    """Live pin in the build container: the same tables from the reference's own ptp_utils / seq_aligner with the real CLIP BPE."""
-    code = r'''
-import sys, gzip, torch
-sys.path.insert(0, %r)
-from oracle import ref_harness as rh
-rh._prepare_imports()
-import video_diffusion.prompt_attention.ptp_utils as rp
-import video_diffusion.prompt_attention.seq_aligner as rs
-from fatezero_b200 import tables
-from transformers import CLIPTokenizer
-lines = gzip.open("/root/reference/CLIP/clip/bpe_simple_vocab_16e6.txt.gz").read().decode("utf-8").split("\n")
-merges = [tuple(m.split()) for m in lines[1:49152 - 256 - 2 + 1]]
-def bytes_to_unicode():
-    bs = list(range(ord("!"), ord("~") + 1)) + list(range(ord("\xa1"), ord("\xac") + 1)) + list(range(ord("\xae"), ord("\xff") + 1))
-    cs = bs[:]
-    n = 0
-    for b in range(2 ** 8):
-        if b not in bs:
-            bs.append(b); cs.append(2 ** 8 + n); n += 1
-    return dict(zip(bs, [chr(c) for c in cs]))
-vocab = list(bytes_to_unicode().values()); vocab = vocab + [v + "</w>" for v in vocab]
-for m in merges: vocab.append("".join(m))
-vocab.extend(["<|startoftext|>", "<|endoftext|>"])
-tok = CLIPTokenizer(vocab=dict(zip(vocab, range(len(vocab)))), merges=merges, model_max_length=77)
-assert tok.encode("a")[1] == 320 and tok.encode("a")[0] == 49406
-pairs = %r
-for src, tgt in pairs:
-    crs = {"default_": 0.8, tgt.split(" ")[1]: 0.3}
-    assert torch.equal(rp.get_time_words_attention_alpha([src, tgt], 50, dict(crs), tok), tables.get_time_words_attention_alpha([src, tgt], 50, dict(crs), tok))
-    m1, a1 = rs.get_refinement_mapper([src, tgt], tok); m2, a2 = tables.get_refinement_mapper([src, tgt], tok)
-    assert torch.equal(m1, m2) and torch.equal(a1, a2)
-    if len(src.split(" ")) == len(tgt.split(" ")):
-        assert torch.equal(rs.get_replacement_mapper([src, tgt], tok), tables.get_replacement_mapper([src, tgt], tok))
-    for w in tgt.split(" "):
-        assert list(rp.get_word_inds(tgt, w, tok)) == list(tables.get_word_inds(tgt, w, tok))
-print("OK")
-''' % (ROOT, PROMPT_PAIRS)
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0 and "OK" in out.stdout, out.stderr[-2000:]
+    """The tables of the reference's own ptp_utils / seq_aligner with the real CLIP BPE (pinned) == this repo's tables."""
+    g = json.load(gzip.open(GOLDEN_TABLES))
+    tok = ReplayTokenizer(g["tokenizer"])
+
+    def ref(name):
+        return torch.tensor(c[name]["data"], dtype=getattr(torch, c[name]["dtype"]))
+
+    assert [(c["source"], c["target"]) for c in g["cases"]] == [tuple(p) for p in PROMPT_PAIRS]
+    for c in g["cases"]:
+        src, tgt = c["source"], c["target"]
+        crs = c["cross_replace_steps"]
+        assert torch.equal(ref("alpha"), tables.get_time_words_attention_alpha([src, tgt], c["num_steps"], dict(crs), tok))
+        m2, a2 = tables.get_refinement_mapper([src, tgt], tok)
+        assert torch.equal(ref("refinement_mapper"), m2) and torch.equal(ref("refinement_alphas"), a2)
+        assert ("replacement_mapper" in c) == (len(src.split(" ")) == len(tgt.split(" ")))
+        if "replacement_mapper" in c:
+            assert torch.equal(ref("replacement_mapper"), tables.get_replacement_mapper([src, tgt], tok))
+        for w in tgt.split(" "):
+            assert list(tables.get_word_inds(tgt, w, tok)) == c["word_inds"][w], (tgt, w)
